@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the learner hot paths named by BASELINE.json.
 
-  python bench.py [--gpus N --steps K --warmup W] [--config cfg2|cfg3|cfg4] [--impl reference]
+  python bench.py [--gpus N --steps K --warmup W] [--config cfg2|cfg3|cfg4] [--impl reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...       (one rank per GPU, NCCL; env-sharded, weak scaling)
 
 Configs (BASELINE.json `configs`):
@@ -313,8 +313,56 @@ def kernel_roofline(name, k, peaks, traffic=None):
     return r
 
 
+# ---------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_ROWS = 1 << 19          # rollout rows written per array: all of cfg2's 524288, a fixed sample of cfg3's 8.4 M
+DUMP_LIMIT = 64 << 20        # bytes over all files
+
+
+def sample_rows(n, device):
+    """Rows of an n-row rollout array that --dump-outputs writes: all of them, or a seeded sample of DUMP_ROWS that is
+    the same in every run, so that two builds can be compared row for row."""
+    import torch
+    if n <= DUMP_ROWS:
+        return slice(None)
+    return torch.from_numpy(np.sort(np.random.RandomState(0).choice(n, DUMP_ROWS, replace=False))).to(device)
+
+
+def seeded_state_restorer(tensors, opt, refresh):
+    """-> a callable that puts the learner back into its state of now (the seeded start): `tensors` (parameters, Adam
+    moments, for deepq the priority trees) get their current values again, the Adam step count goes back, and
+    `refresh` rebuilds what is derived from the parameters.  The gradient, norm and loss reductions of a train step
+    use float atomics, so the state after an update differs in the last bits from run to run, and later updates turn
+    those bits into different sampled actions or replay indices.  --dump-outputs calls it before the last timed step:
+    that step's inputs are then the same in every run, and its outputs differ at most by the rounding of its own
+    reductions."""
+    saved, t = [x.clone() for x in tensors], opt.t
+
+    def restore():
+        for x, s in zip(tensors, saved):
+            x.copy_(s)
+        opt.t = t
+        refresh()
+    return restore
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: tensor or ndarray} as out_dir/<name>.npy.  float64 stays float64, everything else is written as
+    float32 (the integer outputs -- actions, replay indices -- are below 2^24 and stay exact)."""
+    import torch
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        out[name.replace("/", ".").replace(":", "_")] = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the limit of {DUMP_LIMIT}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- PPO2 arm
-def run_ppo2(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx):
+def run_ppo2(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx, dump_dir=None):
     import torch
     import torch.distributed as dist
     from baselines_b200 import _lib
@@ -340,13 +388,16 @@ def run_ppo2(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx):
                       train_chunk=cfg["train_chunk"])
         return model, Runner(env=env, model=model, nsteps=T, gamma=cfg["gamma"], lam=cfg["lam"])
 
+    last = {}
+
     def update(model, runner):
         ro, _ = runner.run_device()
         st = run_epochs(model, ro, cfg["lr"], cfg["cliprange"], nbatch, nbatch_train, cfg["noptepochs"], dev,
                         shuffle=args.shuffle)
+        last["stats"] = st
         return torch.stack(st).mean(dim=0)
 
-    def timed(model, runner, steps, warmup, read_back, profile=False):
+    def timed(model, runner, steps, warmup, read_back, profile=False, before_last=None):
         for _ in range(warmup):
             update(model, runner)
         torch.cuda.synchronize()
@@ -355,30 +406,50 @@ def run_ppo2(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        l0 = _lib.LAUNCHES
-        e0.record()
-        for _ in range(steps):
-            st = update(model, runner)
-            if read_back:
-                st.cpu()                                         # the loss statistics a user reads each update
-        e1.record()
-        torch.cuda.synchronize()
+        ms, launches = 0.0, 0
+        for i, n in enumerate([steps] if before_last is None else [steps - 1, 1]):
+            if i == 1:                                           # between the two timed windows
+                before_last()
+                torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            l0 = _lib.LAUNCHES
+            e0.record()
+            for _ in range(n):
+                st = update(model, runner)
+                if read_back:
+                    st.cpu()                                     # the loss statistics a user reads each update
+            e1.record()
+            torch.cuda.synchronize()
+            ms += e0.elapsed_time(e1)
+            launches += _lib.LAUNCHES - l0
         if world > 1:
             dist.barrier()
-        ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+        ms = torch.tensor([ms], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()) / steps, (_lib.LAUNCHES - l0) / steps
+        return float(ms.item()) / steps, launches / steps
 
     # ---- device-resident value: first un-instrumented (the headline), then once more with per-call CUDA events
     env_d = DeviceSyntheticVecEnv(N, cfg["ob_shape"], ob_dtype, seed=rank, device=dev, **env_kw)
     model, runner = make(env_d)
+    reseed = None
+    if dump_dir:
+        store = model.net.store
+        reseed = seeded_state_restorer([store.params, store.m, store.v], model.opt, model.net.refresh)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_step, launches = timed(model, runner, steps, warmup, read_back=False)
+    ms_step, launches = timed(model, runner, steps, warmup, read_back=False, before_last=reseed)
     clocks = sampler.stop() if rank == 0 else None
+    if dump_dir and rank == 0:
+        st = torch.stack(last["stats"])
+        out = {"loss_stats": st.mean(dim=0), "loss_stats_per_minibatch": st,
+               "last_values": runner.rollout.last_values}
+        rows = sample_rows(nbatch, dev)
+        for name in ("actions", "values", "neglogpacs", "advs", "returns"):
+            out["rollout_" + name] = runner.rollout.flat(name)[rows]
+        out.update(("params." + k, v) for k, v in model.get_params().items())
+        dump_outputs(dump_dir, out)
     prof = None
     ms_prof = None
     if with_profile:
@@ -437,7 +508,7 @@ def run_ppo2(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx):
 
 
 # ---------------------------------------------------------------------------------------------- deepq arm
-def run_deepq(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx):
+def run_deepq(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx, dump_dir=None):
     import random
     import torch
     from baselines_b200 import _lib
@@ -464,31 +535,51 @@ def run_deepq(cfg, args, steps, warmup, with_profile, with_e2e, dist_ctx):
     rb._set_priorities(torch.arange(n_fill, device=dev), pr)
     torch.cuda.synchronize()
 
+    last = {}
+
     def step():
         idx, w32, _ = rb.sample_device(B, beta=cfg["beta"])
         td = model.train_device(rb._obs_t, rb._obs_tp1, rb._actions, rb._rewards, rb._dones, w32, idx, B)
         rb.update_priorities_device(idx, td, 1e-6)
+        last.update(sample_idx=idx, sample_weights=w32, td_errors=td)
 
-    def timed(fn, steps, warmup, profile=False):
+    def timed(fn, steps, warmup, profile=False, before_last=None):
         for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
         if profile:
             _lib.profile_begin()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        l0 = _lib.LAUNCHES
-        e0.record()
-        for _ in range(steps):
-            fn()
-        e1.record()
-        torch.cuda.synchronize()
-        return e0.elapsed_time(e1) / steps, (_lib.LAUNCHES - l0) / steps
+        ms, launches = 0.0, 0
+        for i, n in enumerate([steps] if before_last is None else [steps - 1, 1]):
+            if i == 1:                                           # between the two timed windows
+                before_last()
+                torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            l0 = _lib.LAUNCHES
+            e0.record()
+            for _ in range(n):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            ms += e0.elapsed_time(e1)
+            launches += _lib.LAUNCHES - l0
+        return ms / steps, launches / steps
 
+    reseed = None
+    if dump_dir:
+        q = model.q.store
+        reseed = seeded_state_restorer([q.params, q.m, q.v, rb._it_sum, rb._it_min, rb._maxp_dev], model.opt,
+                                       model.q.refresh)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_step, launches = timed(step, steps, warmup)
+    ms_step, launches = timed(step, steps, warmup, before_last=reseed)
     clocks = sampler.stop() if rank == 0 else None
+    if dump_dir and rank == 0:
+        out = dict(last)
+        out["priorities"] = rb._it_sum[rb._cap + last["sample_idx"]]          # the leaves the step rewrote
+        out.update(("params." + k, v) for k, v in model.q.store.export_tf("params").items())
+        dump_outputs(dump_dir, out)
     prof = None
     if with_profile:
         timed(step, 20, 0, profile=True)
@@ -546,6 +637,9 @@ def main():
     ap.add_argument("--no-profile", action="store_true", help="skip the per-kernel CUDA-event profile pass")
     ap.add_argument("--no-targets", action="store_true", help="skip the stand-alone GAE / fc1 / PER microbenchmarks")
     ap.add_argument("--no-others", action="store_true", help="default config only: skip the short cfg3 / cfg4 measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (at most 64 MB); that step starts from "
+                         "the learner's seeded state, so its inputs are the same in every run")
     args = ap.parse_args()
     cfg = dict(CFGS[args.config])
     if args.nenvs and cfg["kind"] == "ppo2":
@@ -554,6 +648,10 @@ def main():
         args.steps = cfg["steps"]
     if args.warmup is None:
         args.warmup = cfg["warmup"]
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.impl == "reference":
         return run_reference(args, cfg)
 
@@ -572,7 +670,7 @@ def main():
         dist.barrier()
     ctx = (rank, local_rank, world)
     runner_fn = run_deepq if cfg["kind"] == "deepq" else run_ppo2
-    res = runner_fn(cfg, args, args.steps, args.warmup, not args.no_profile, not args.no_e2e, ctx)
+    res = runner_fn(cfg, args, args.steps, args.warmup, not args.no_profile, not args.no_e2e, ctx, args.dump_outputs)
 
     # short, driver-visible measurements of the other BASELINE configs (N = 1 only: they are single-GPU configs)
     others = None
